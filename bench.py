@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port) on the host cores
     python bench.py --impl cudnn ...                         # the same graph on PyTorch/cuDNN CUDA kernels ("reference CUDA" row)
     python bench.py --config generator|vtoonify_t|video ...  # BASELINE configs[2] / [4] / [3]
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's output to DIR (dump_outputs)
 
 Default (configs[1]): a "step" is one ``VToonify.forward`` (+ clamp) over one batch of 4 synthetic 576x1024 frames per GPU
 (VToonify-D, deterministic random-init weights).
@@ -355,6 +356,37 @@ def _roofline(prof, steps, ms, precision, peaks, cfg, units_per_rank_step, extra
     return roof, per
 
 
+DUMP_BYTES = 64 << 20              # --dump-outputs writes at most this much in all
+DUMP_SAMPLE = 1 << 22              # at most this many float32 values per output (16 MB)
+DUMP_SEED = 0
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each named output tensor as ``<out_dir>/<name>.npy`` (float32).  An output of more than DUMP_SAMPLE values is
+    written as its values at DUMP_SAMPLE flat indices drawn from DUMP_SEED (sorted, duplicates dropped): the same indices for
+    the same shape, so two builds can be compared value for value.  ``<name>_stats.npy`` (float64: numel, sum, sum of
+    squares, min, max over the whole tensor) goes with each.  Returns the description for the JSON line."""
+    import numpy as np
+    import torch
+    assert len(outputs) * (DUMP_SAMPLE * 4 + 4096) <= DUMP_BYTES, "too many outputs for the --dump-outputs budget"
+    os.makedirs(out_dir, exist_ok=True)
+    desc = {}
+    for name, t in outputs.items():
+        t = t.detach().float().reshape(-1)
+        d = t.double()
+        stats = np.array([t.numel(), d.sum().item(), d.square().sum().item(), d.min().item(), d.max().item()], dtype=np.float64)
+        if t.numel() <= DUMP_SAMPLE:
+            vals, how = t.reshape(outputs[name].shape).cpu().numpy(), "whole"
+        else:
+            idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, t.numel(), DUMP_SAMPLE))
+            vals = t[torch.from_numpy(idx).to(t.device)].cpu().numpy()
+            how = f"{vals.size} values at flat indices np.unique(default_rng({DUMP_SEED}).integers(0, {t.numel()}, {DUMP_SAMPLE}))"
+        np.save(os.path.join(out_dir, name + ".npy"), vals.astype(np.float32))
+        np.save(os.path.join(out_dir, name + "_stats.npy"), stats)
+        desc[name] = {"shape": list(outputs[name].shape), "written": how}
+    return {"dir": os.path.abspath(out_dir), "outputs": desc}
+
+
 def run_ours(args, cfg, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -420,8 +452,9 @@ def run_ours(args, cfg, rank, world, local_rank):
             ops.set_tc_profile(prof)
             n0 = _lib.launch_count()
             e0.record()
-            for _ in range(steps):
+            for _ in range(steps - 1):
                 step()
+            out = step()                                         # the last step's result, for --dump-outputs
             e1.record()
             barrier()
         else:
@@ -447,6 +480,8 @@ def run_ours(args, cfg, rank, world, local_rank):
         ops.set_tc_profile(None)
         ms = e0.elapsed_time(e1)
         clocks = sampler.stop() if sampler else None
+        dumped = dump_outputs(args.dump_outputs, {"images" if is_gen else "frames": out}) if args.dump_outputs else None
+        out = None                                               # not held through the end-to-end legs
 
         # ---- e2e through the public frame-loop API with host buffers
         e2e = e2e_u8 = None
@@ -549,6 +584,8 @@ def run_ours(args, cfg, rank, world, local_rank):
     if world == 1 and not args.no_cpu_baseline:
         _, _, cb = cpu_reference(cfg, 1, 0)
         line["cpu_baseline"] = cb
+    if dumped:
+        line["dump_outputs"] = dumped
     emit(json.dumps(line))
 
 
@@ -688,7 +725,14 @@ def main():
     ap.add_argument("--ref-budget", type=float, default=660.0,
                     help="--impl reference: seconds the K timed CPU steps may take; full-size frames unless the host is too slow for that")
     ap.add_argument("--no-u8", action="store_true", help="skip the uint8-wire / on-device parsing end-to-end leg")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32; a fixed seeded "
+                         "sample of an output above 4M values) to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config == "video" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs covers the single-process timed step of --impl ours (not --config video)")
     cfg = dict(CONFIGS[args.config])
     if args.backbone:
         cfg["backbone"] = args.backbone

@@ -1,11 +1,27 @@
-"""Shared test helpers: rebuild the deterministic state_dicts of the single-layer golden fixtures without the
-reference (shapes are those of the reference constructors used in tests/golden/make_golden.py)."""
+"""Shared test helpers: rebuild what the golden fixtures do not store, without the reference: the deterministic
+state_dicts of the single-layer fixtures (shapes are those of the reference constructors used in
+tests/golden/make_golden.py) and the input frames of the VToonify fixtures."""
+import os
+
+import numpy as np
 import torch
 
 from oracle import vt_oracle as O
-from vtoonify_b200.weights import det_state_dict
+from vtoonify_b200.weights import det_inputs, det_state_dict
 
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 K4 = O.make_kernel([1, 3, 3, 1])
+VTOONIFY_CASES = {"a": (2, 32, 32), "b": (1, 48, 40)}      # (B, H, W) of the vtoonify_{d,t} golden cases
+
+
+def vtoonify_frames(g, case):
+    """Input frame batch ``x`` of a vtoonify_{d,t} golden case, redrawn from the seed make_golden.py used; the fixture
+    keeps every 16th value of it to check the redraw."""
+    B, H, W = VTOONIFY_CASES[case]
+    x = det_inputs(B, H, W, seed=ord(case))[0]
+    assert np.array_equal(x.reshape(-1)[::16].numpy(), g[f"{case}_x_every16"]), \
+        f"det_inputs no longer redraws the frames of golden case {case}"
+    return x
 
 
 def _styled_conv_template(cin, cout, up):

@@ -1,10 +1,13 @@
 """GPU parity of the pSp style encoder (SURVEY §8 row a10) against the reference output in tests/golden/psp.npz."""
 import json
+import os
 from argparse import Namespace
 
 import numpy as np
 import pytest
 import torch
+
+from tests.shapes import GOLDEN
 
 pytestmark = pytest.mark.gpu
 torch.set_grad_enabled(False)
@@ -17,7 +20,7 @@ def test_psp_encoder(golden, prec, tol):
     from vtoonify_b200.weights import det_state_dict
     g = golden("psp")
     m = GradualStyleEncoder(50, "ir_se", Namespace(input_nc=3, n_styles=18)).eval()
-    keys = json.load(open("tests/golden/state_dict_keys_psp.json"))
+    keys = json.load(open(os.path.join(GOLDEN, "state_dict_keys_psp.json")))
     sd = m.state_dict()
     assert list(sd.keys()) == list(keys.keys()) and all(list(sd[k].shape) == keys[k] for k in keys)
     m.load_state_dict(det_state_dict(m, seed=11), strict=True)

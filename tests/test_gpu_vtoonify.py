@@ -1,9 +1,12 @@
 """GPU parity of VToonify.forward (D and T backbones) against the reference outputs in tests/golden."""
 import json
+import os
 
 import numpy as np
 import pytest
 import torch
+
+from tests.shapes import GOLDEN, vtoonify_frames
 
 pytestmark = pytest.mark.gpu
 torch.set_grad_enabled(False)
@@ -22,7 +25,7 @@ def model(request):
     from vtoonify_b200.weights import det_state_dict
     backbone = {"d": "dualstylegan", "t": "toonify"}[request.param]
     m = VToonify(backbone=backbone).eval()
-    keys = json.load(open(f"tests/golden/state_dict_keys_{request.param}.json"))
+    keys = json.load(open(os.path.join(GOLDEN, f"state_dict_keys_{request.param}.json")))
     sd = m.state_dict()
     assert list(sd.keys()) == list(keys.keys())
     assert all(list(sd[k].shape) == keys[k] for k in keys)
@@ -38,7 +41,7 @@ def test_forward_golden(golden, model, prec):
     ops.set_precision(prec)
     try:
         for case in ("a", "b"):
-            x, style = T(g[f"{case}_x"]).cuda(), T(g[f"{case}_style"]).cuda()
+            x, style = vtoonify_frames(g, case).cuda(), T(g[f"{case}_style"]).cuda()
             if tag == "d":
                 y, masks = m(x, style, d_s=0.5, return_mask=True)
                 for i, mk in enumerate(masks):
@@ -61,14 +64,14 @@ def test_aux_paths(golden, model):
     g = golden(f"vtoonify_{tag}")
     w = m.zplus2wplus(T(g["zplus"]).cuda())
     assert (w.cpu() - T(g["wplus"])).abs().max().item() <= 5e-5
-    x, style = T(g["b_x"]).cuda(), T(g["b_style"]).cuda()
+    x, style = vtoonify_frames(g, "b").cuda(), T(g["b_style"]).cuda()
     feat, skip = m(x, style, d_s=0.5, return_feat=True)
     assert feat.shape == (1, 512, 6, 5) and skip.shape == (1, 3, 6, 5)
     # 2-D style ([B, 512]) path of forward (model/vtoonify.py:212-216)
     y = m(x, style[:, 0], d_s=0.5)
     assert y.shape == (1, 3, 192, 160) and torch.isfinite(y).all()
     # batch independence: frames are independent units (multi-GPU sharding relies on it)
-    xa, sa = T(g["a_x"]).cuda(), T(g["a_style"]).cuda()
+    xa, sa = vtoonify_frames(g, "a").cuda(), T(g["a_style"]).cuda()
     y2 = m(xa, sa, d_s=0.5)
     y0 = m(xa[:1], sa[:1], d_s=0.5)
     assert (y2[:1] - y0).abs().max().item() <= 1e-5
@@ -81,7 +84,7 @@ def test_style_cache(golden, model):
     from vtoonify_b200.weights import det_state_dict
     tag, m = model
     g = golden(f"vtoonify_{tag}")
-    x = T(g["a_x"]).cuda()                                           # B = 2
+    x = vtoonify_frames(g, "a").cuda()                                         # B = 2
     style = T(g["a_style"])[:1].repeat(2, 1, 1).cuda()              # one video, one style: both rows carry the same code
     y_first = m(x, style, d_s=0.5)
     n0 = _lib.launch_count()

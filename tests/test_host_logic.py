@@ -164,7 +164,7 @@ def test_bisenet_state_dict_keys_and_host_algebra():
     from vtoonify_b200.bisenet import BiSeNet, S2D_TAPS, fold_bn, s2d_stem_weight
     from vtoonify_b200.psp import BatchNorm2d
     m = BiSeNet(19)
-    keys = json.load(open("tests/golden/state_dict_keys_bisenet.json"))
+    keys = json.load(open(os.path.join(ROOT, "tests", "golden", "state_dict_keys_bisenet.json")))
     sd = m.state_dict()
     assert list(sd.keys()) == list(keys.keys()) and all(list(sd[k].shape) == keys[k] for k in keys)
 

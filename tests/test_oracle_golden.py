@@ -1,6 +1,7 @@
 """CPU: pin oracle/vt_oracle.py against outputs of the unmodified reference (tests/golden/*.npz, produced by
-tests/golden/make_golden.py from /root/reference's op_cpu path)."""
+tests/golden/make_golden.py from the reference's op_cpu path)."""
 import json
+import os
 
 import numpy as np
 import pytest
@@ -8,7 +9,7 @@ import torch
 
 from oracle import vt_oracle as O
 from vtoonify_b200.weights import det_state_dict
-from tests.shapes import layer_state_dict
+from tests.shapes import GOLDEN, layer_state_dict, vtoonify_frames
 
 torch.set_grad_enabled(False)
 
@@ -91,14 +92,14 @@ def test_generator_golden(golden):
 @pytest.mark.parametrize("tag,backbone", [("d", "dualstylegan"), ("t", "toonify")])
 def test_vtoonify_golden(golden, tag, backbone):
     g = golden(f"vtoonify_{tag}")
-    keys = json.load(open(f"tests/golden/state_dict_keys_{tag}.json"))
+    keys = json.load(open(os.path.join(GOLDEN, f"state_dict_keys_{tag}.json")))
     sd = det_state_dict({k: torch.empty(v) for k, v in keys.items()}, seed=0)
     # FIR buffers are architecture constants, not random (weights.py keeps the template value)
     for k in sd:
         if k.endswith("blur.kernel") or k.endswith("upsample.kernel"):
             sd[k] = O.make_kernel([1, 3, 3, 1]) * 4
     for case in ("a", "b"):
-        x, style = T(g[f"{case}_x"]), T(g[f"{case}_style"])
+        x, style = vtoonify_frames(g, case), T(g[f"{case}_style"])
         if backbone == "dualstylegan":
             y, masks = O.vtoonify_forward(sd, x, style, 0.5, backbone, return_mask=True)
             for i, m in enumerate(masks):
@@ -125,7 +126,7 @@ def test_frame_transforms():
 def test_psp_encoder_golden(golden):
     """a10: pSp GradualStyleEncoder(50, 'ir_se') restated functionally vs the reference module's output."""
     g = golden("psp")
-    keys = json.load(open("tests/golden/state_dict_keys_psp.json"))
+    keys = json.load(open(os.path.join(GOLDEN, "state_dict_keys_psp.json")))
     sd = det_state_dict({k: torch.empty(v, dtype=torch.long if k.endswith("num_batches_tracked") else torch.float32)
                          for k, v in keys.items()}, seed=11)
     y = O.psp_forward(sd, T(g["x"]).float())
@@ -137,7 +138,7 @@ def test_bisenet_parsing_golden(golden):
     """Next row (f): BiSeNet parsing maps of the frame loop (2x bilinear up-sampling, BiSeNet, nearest back to frame size),
     restated functionally from the state_dict, vs the reference module's output."""
     g = golden("bisenet")
-    keys = json.load(open("tests/golden/state_dict_keys_bisenet.json"))
+    keys = json.load(open(os.path.join(GOLDEN, "state_dict_keys_bisenet.json")))
     sd = det_state_dict({k: torch.empty(v, dtype=torch.long if k.endswith("num_batches_tracked") else torch.float32)
                          for k, v in keys.items()}, seed=21)
     y = O.parsing_for_vtoonify(sd, T(g["x"]).float())
